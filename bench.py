@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload resnet|microbench] [--per-domain B] [--site-mode fused|modules]
+                    [--dump-outputs DIR]
 
 One "step" = one full training step of the ResNet-50-DWT harness model (harness/resnet50_dwt.py,
 the reference topology with this repo's CUDA layers dropped in) on one synthetic Office-Home-shaped
@@ -27,6 +28,9 @@ At N = 1 the line also carries
 --impl reference: the reference's own CPU path (no GPU): the same step with the reference's
 operator sequence on stock ATen CPU ops (oracle/torch_port.py), all host threads, a bounded sample.
 --workload microbench: only BASELINE.json configs[1] (WTransform2d N=256 C=256 56x56 gs=64 fwd+bwd).
+--dump-outputs DIR: after the K timed steps, DIR/{loss,logits,param_grads,params,buffers}.npy hold what the last
+of them computed (dump_outputs()).  That step starts from the seeded checkpoint again (restored outside the timed
+window), on the seeded batch: every run, whatever K and W, dumps one training step from the same inputs.
 """
 from __future__ import annotations
 
@@ -269,7 +273,7 @@ class FlatGradAllReduce:
 
 
 def train_step(model, mec, opt, images, labels, sync=None, head=None):
-    """head: dwt_b200.HeadLoss -- the same NLL + lambda*MEC as one fused launch (GPU arm)."""
+    """-> (loss, logits).  head: dwt_b200.HeadLoss -- the same NLL + lambda*MEC as one fused launch (GPU arm)."""
     if sync is None:
         opt.zero_grad(set_to_none=True)
     else:
@@ -284,7 +288,32 @@ def train_step(model, mec, opt, images, labels, sync=None, head=None):
     if sync is not None:
         sync.reduce()
     opt.step()
-    return loss
+    return loss, logits
+
+
+DUMP_SAMPLE = 1 << 21                            # elements kept of each flattened parameter-sized output
+
+
+def dump_outputs(out_dir, model, loss, logits):
+    """Write what one training step hands back to its caller as float32 .npy files: the loss and the logits whole;
+    the parameter gradients, the updated parameters and the running statistics flattened in named_parameters /
+    named_buffers order (logical NCHW order whatever the memory format), the first two as a fixed seeded sample of
+    DUMP_SAMPLE of their 23.6 M elements -- the same elements in every run, so two builds compare output for output.
+    Two runs of one build with the same arguments write bit-identical files (NVIDIA B200, 1000 W power limit)."""
+    import numpy as np
+    params = [p for _, p in model.named_parameters()]
+    flat = {"param_grads": torch.cat([p.grad.reshape(-1) for p in params]),
+            "params": torch.cat([p.detach().reshape(-1) for p in params]),
+            "buffers": torch.cat([b.reshape(-1).float() for _, b in model.named_buffers()])}
+    arrays = {"loss": loss.detach(), "logits": logits.detach()}
+    for name, v in flat.items():
+        if v.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(v.numel(), DUMP_SAMPLE, replace=False))
+            v = v[torch.from_numpy(idx).to(v.device)]
+        arrays[name] = v
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v.float().cpu().numpy())
 
 
 # ----------------------------------------------------------------------------------------- arms
@@ -458,18 +487,25 @@ def reference_on_gpu_micro(args, device):
                     "grouped conv2d; autograd backward), eager, fp32"}
 
 
-def timed_loop(step_fn, steps, device, distributed):
+def timed_loop(step_fn, steps, device, distributed, before_last=None):
+    """Device time of `steps` calls of step_fn.  before_last (optional) runs between the last two steps, outside the
+    timed window."""
     import torch.distributed as dist
     if distributed:
         dist.barrier()
     torch.cuda.synchronize(device)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(steps):
+    for i in range(steps):
+        if before_last is not None and i == steps - 1:
+            p0.record()
+            before_last()
+            p1.record()
         step_fn()
     e1.record()
     torch.cuda.synchronize(device)
-    ms = torch.tensor([e0.elapsed_time(e1)], device=device)
+    ms = torch.tensor([e0.elapsed_time(e1) - (p0.elapsed_time(p1) if before_last is not None else 0.0)], device=device)
     if distributed:
         dist.barrier()
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -512,7 +548,11 @@ def run_ours(args):
             os.dup2(saved, 1)
             os.close(saved)
     assert world == args.gpus, f"--gpus {args.gpus} but WORLD_SIZE={world}"
-    torch.backends.cudnn.benchmark = True
+    # cuDNN's heuristics choose the convolution algorithms from the shapes alone.  Autotuning (benchmark=True) chooses by
+    # timing, so two runs could take different TF32 algorithms and compute different results: the training step turns
+    # that rounding into several % of the gradients.  The fixed choice costs ~0.9 ms per step (29.7 vs 28.8 ms with
+    # autotuning, NVIDIA B200 at 1000 W), most of it in the stem convolution.
+    torch.backends.cudnn.benchmark = False
     _native.lib()                                           # fail loudly if the extension is missing
 
     if args.workload == "microbench":
@@ -536,6 +576,16 @@ def run_ours(args):
     net = model
     sync = FlatGradAllReduce(model, world, segments=args.grad_segments, gather=args.grad_gather) if distributed else None   # one GPU: plain .grad tensors
     opt = make_optimizer(model)
+    # --dump-outputs: the last timed step starts again from the seeded checkpoint (weights and running statistics as
+    # built, momentum buffers zero = a fresh SGD), so what it computes does not depend on the steps before it.  Training
+    # on one fixed synthetic batch is chaotic -- a 1e-6 change of one weight reaches several % of the logits within
+    # three steps -- so otherwise a cuDNN algorithm choice or a reordered sum decides what the dump holds.
+    seeded = [t.detach().clone() for t in model.state_dict().values()] if args.dump_outputs else None
+
+    def restore_seeded():
+        torch._foreach_copy_(list(model.state_dict().values()), seeded)
+        torch._foreach_zero_([s["momentum_buffer"] for s in opt.state.values()])
+
     mec = dwt_b200.MinEntropyConsensusLoss(NUM_CLASSES, device)
     head = dwt_b200.HeadLoss(NUM_CLASSES, LAMBDA_MEC)
     B = args.per_domain
@@ -545,14 +595,16 @@ def run_ours(args):
     host_images, host_labels = host_images.pin_memory(), host_labels.pin_memory()
     images, labels = host_images.to(device), host_labels.to(device)
     loss_host = torch.zeros((), dtype=torch.float32).pin_memory()
+    last = {}                                               # (loss, logits) of the latest eager step, detached: a
+                                                            # live autograd graph would break the CUDA-graph capture
 
     def step_resident():
-        train_step(net, mec, opt, images, labels, sync, head)
+        last["out"] = tuple(t.detach() for t in train_step(net, mec, opt, images, labels, sync, head))
 
     def step_e2e():
         im = host_images.to(device, non_blocking=True)
         lb = host_labels.to(device, non_blocking=True)
-        loss = train_step(net, mec, opt, im, lb, sync, head)
+        loss, _ = train_step(net, mec, opt, im, lb, sync, head)
         loss_host.copy_(loss.detach(), non_blocking=True)
         torch.cuda.current_stream(device).synchronize()     # the user reads the loss every step
 
@@ -569,7 +621,7 @@ def run_ours(args):
 
     # Pass 2: the same step captured once into a CUDA graph and replayed (the step is ~1400 launches, the
     # host launch path is as long as the GPU work).  This is the reported `value`; identical kernels and work.
-    graph, static_loss = None, None
+    graph, static_loss, static_logits = None, None, None
     if args.cuda_graph:
         try:
             side = torch.cuda.Stream(device)
@@ -581,7 +633,7 @@ def run_ours(args):
             torch.cuda.synchronize(device)
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                static_loss = train_step(net, mec, opt, images, labels, sync, head)
+                static_loss, static_logits = train_step(net, mec, opt, images, labels, sync, head)
             torch.cuda.synchronize(device)
         except Exception as e:                      # capture is an optimisation, never a requirement
             graph = None
@@ -617,7 +669,9 @@ def run_ours(args):
     for _ in range(2):
         step_timed()
     with ClockSampler(local) as clocks:
-        ms = timed_loop(step_timed, args.steps, device, distributed)
+        ms = timed_loop(step_timed, args.steps, device, distributed, before_last=restore_seeded if args.dump_outputs else None)
+    if args.dump_outputs and rank == 0:                    # before the e2e passes below train the model further
+        dump_outputs(args.dump_outputs, model, *((static_loss, static_logits) if graph is not None else last["out"]))
     for _ in range(2):
         step_e2e()
     ms_e2e = timed_loop(step_e2e, args.steps, device, distributed)
@@ -730,14 +784,15 @@ def run_ours(args):
         "gpu_launches": int(launches), "clocks": clocks.summary(), "roofline": roof, "kernels": fams,
         "e2e_uint8_input": e2e_u8,
         "cuda_graph": graph is not None, "eager_ms_per_step": ms_eager / args.steps,
-        "conv_math": "cuDNN, TF32 allowed (torch default) -- convolutions are not part of the hot path",
+        "conv_math": "cuDNN, TF32 allowed (torch default), algorithms chosen by cuDNN's heuristics (no autotuning) -- "
+                     "convolutions are not part of the hot path",
     }
     if args.cpu_baseline:
         out["cpu_baseline"] = cpu_baseline(args)
     out["status_word"] = _native.status_all(device)            # 0: no kernel reported a failure during the run
     if not distributed and args.extras:
         # free the step's graph, model and activations before the two side measurements
-        del graph, static_loss, model, net, opt
+        del graph, static_loss, static_logits, last, seeded, model, net, opt
         import gc
         gc.collect()
         torch.cuda.empty_cache()
@@ -869,7 +924,13 @@ def main():
                     help="pieces the flat gradient buffer is all-reduced in (1 = one collective after backward)")
     ap.add_argument("--micro-n", type=int, default=256)
     ap.add_argument("--micro-gs", type=int, default=64)
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last timed training step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "resnet"):
+        ap.error("--dump-outputs writes the outputs of the ResNet-50-DWT training step: --impl ours --workload resnet")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":
